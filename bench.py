@@ -7,8 +7,10 @@ One "step" = one pass of the hot path over one batch: prefill of B x 1024 prompt
     python bench.py --gpus 1 --steps 5 --warmup 3              # this repo's CUDA path
     python bench.py --impl reference --gpus 1 --steps 2        # the reference's HF-transformers CPU backend
     torchrun --nproc-per-node N ... bench.py --gpus N ...      # TP=N over NCCL
+    python bench.py --gpus 1 --steps 5 --dump-outputs DIR      # also save the last timed step's output ids
 
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for how each field is obtained.
+Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for how each field is obtained.  Writes nothing into the
+source tree, which may be read-only.
 """
 from __future__ import annotations
 
@@ -23,6 +25,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ from the imports below: the tree is left as the build left it
 
 LLAMA3_8B = dict(vocab_size=128256, hidden_size=4096, intermediate_size=14336, num_hidden_layers=32,
                  num_attention_heads=32, num_key_value_heads=8, head_dim=128, max_position_embeddings=8192,
@@ -404,8 +407,10 @@ def run_b200(args):
     wall = time.perf_counter() - t_wall0
     launches = eng.last_launches()
     clocks = sampler.stop() if rank == 0 else None
-    out = eng.fetch_staged()
+    out = eng.fetch_staged()            # every timed step replays the staged prompt: these are the last step's ids
     assert out.shape == (B, S + T), out.shape
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"output_ids": out})
     dev_ms = sum(pre) + sum(dec)
     tm = torch.tensor([dev_ms, statistics.median(pre), sum(dec)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -519,6 +524,22 @@ def run_b200(args):
     emit(line)
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: what the timed path handed its caller, as DIR/<name>.npy in float64 (exact for token ids).  The
+    prompt and the weights are seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    host = {name: t.cpu().numpy().astype(np.float64) for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _REAL_STDOUT = None
 
 
@@ -547,7 +568,13 @@ def main():
                     help="--impl reference: CPU seconds the whole --steps/--warmup run may take before the sample is shortened")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity-check", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output ids of the last timed step to DIR/output_ids.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path, not --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -3,6 +3,10 @@ import json
 import os
 import sys
 
+import numpy as np
+import pytest
+import torch
+
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench  # noqa: E402
 
@@ -35,6 +39,17 @@ def test_cpu_thread_policy_and_peaks():
     p = bench.load_peaks()
     assert p["hbm_gbs"] > 1000 and p["tf_sustained"] <= p["tf_burst"]
     assert json.dumps(p)
+
+
+def test_dump_outputs_writes_exact_float64_ids(tmp_path, monkeypatch):
+    ids = torch.randint(0, 128256, (4, 9), generator=torch.Generator().manual_seed(0), dtype=torch.int64)
+    bench.dump_outputs(str(tmp_path / "out"), {"output_ids": ids})
+    a = np.load(tmp_path / "out" / "output_ids.npy")
+    assert a.dtype == np.float64 and a.shape == (4, 9) and np.array_equal(a.astype(np.int64), ids.numpy())
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", ids.numel() * 8 - 1)
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "big"), {"output_ids": ids})
+    assert not (tmp_path / "big").exists()
 
 
 def test_both_arms_share_one_config_dict():
