@@ -172,15 +172,12 @@ int b200_op_gemm(const void* A, const void* B, void* out, const void* residual, 
                  int block_n, int splits, int64_t ldo, void* stream);
 int b200_op_rmsnorm(void* x, const void* w, void* xn, int rows, int H, float eps, const float* partial,
                     int splits, const void* y, void* stream);
-int b200_op_attn_prefill(const void* q, int64_t ldq, void* out, int64_t ldo, const void* kcache,
-                         const void* vcache, const int32_t* page_table, int max_pages,
-                         const int32_t* cu_seqlens, const int32_t* seq_slot, int B, int max_len, int nh, int nkv,
-                         void* stream);
-/* tcgen05/TMEM prefill attention (the engine's default); q_rows = rows of the q buffer, num_pages = pages of the caches */
+/* tcgen05/TMEM prefill attention (the engine's); q_rows = rows of the q buffer, num_pages = pages of the caches */
 int b200_op_attn_prefill_tc(const void* q, int64_t ldq, int q_rows, void* out, int64_t ldo, const void* kcache,
                             const void* vcache, int num_pages, const int32_t* page_table, int max_pages,
                             const int32_t* cu_seqlens, const int32_t* seq_slot, int B, int max_len, int nh, int nkv,
                             void* stream);
+/* split-KV decode attention; with splits > 1 the last CTA of each (row, kv head) merges the part_o / part_ml partials */
 int b200_op_attn_decode(const void* q, int64_t ldq, void* out, int64_t ldo, const void* kcache,
                         const void* vcache, const int32_t* page_table, int max_pages, const int32_t* seq_slot,
                         const int32_t* tok_pos, int B, int nh, int nkv, int splits, float* part_o, float* part_ml,

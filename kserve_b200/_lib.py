@@ -67,8 +67,6 @@ def load() -> C.CDLL:
     lib.b200_fetch_staged.argtypes = [vp, vp, C.POINTER(i32), C.POINTER(i32)]
     lib.b200_op_gemm.argtypes = [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, i64, vp]
     lib.b200_op_rmsnorm.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_float, vp, C.c_int, vp, vp]
-    lib.b200_op_attn_prefill.argtypes = [vp, i64, vp, i64, vp, vp, vp, C.c_int, vp, vp, C.c_int, C.c_int,
-                                         C.c_int, C.c_int, vp]
     lib.b200_op_attn_prefill_tc.argtypes = [vp, i64, C.c_int, vp, i64, vp, vp, C.c_int, vp, C.c_int, vp, vp, C.c_int, C.c_int,
                                             C.c_int, C.c_int, vp]
     lib.b200_op_attn_decode.argtypes = [vp, i64, vp, i64, vp, vp, vp, C.c_int, vp, vp, C.c_int, C.c_int,

@@ -1,14 +1,14 @@
-// Attention over the paged KV cache (SURVEY.md §8a row 15: LlamaAttention.forward + SDPA with GQA).
+// Decode attention over the paged KV cache (SURVEY.md §8a row 15: LlamaAttention.forward + SDPA with GQA); the
+// prefill attention is the tcgen05 kernel in attention_tc.cuh.
 //
-//   attn_prefill_kernel : causal flash attention for the prompt tokens of ragged sequences.
-//   attn_decode_kernel  : one query token per sequence, split over the KV length (flash-decoding),
-//                         the G query heads that share a KV head are packed into the MMA M dimension.
-//   attn_combine_kernel : merges the per-split partials.
+//   attn_decode_kernel : one query token per sequence, split over the KV length (flash-decoding),
+//                        the G query heads that share a KV head are packed into the MMA M dimension;
+//                        the last split CTA to arrive merges the per-split partials.
 //
 // KV pages are [page][kv_head][64 tokens][128 dims] bf16, so one (page, kv_head) tile is a contiguous
 // 16 KB block that is staged with 128-bit cp.async into XOR-swizzled shared memory and consumed with
-// ldmatrix + mma.sync.m16n8k16 (fp32 softmax / accumulation).  This round's kernels use the legacy
-// warp-level MMA path; they are HBM-bound in decode (the KV read) and 2% of prefill FLOPs.
+// ldmatrix + mma.sync.m16n8k16 (fp32 softmax / accumulation).  The warp-level MMA path suffices here: the
+// kernel is HBM-bound (the KV read).
 #pragma once
 #include "common.cuh"
 #include "ops.cuh"
@@ -32,159 +32,6 @@ __device__ __forceinline__ void load_kv_tile(uint32_t sdst, const bf16* gsrc) {
   }
 }
 
-struct AttnPrefillParams {
-  const bf16* q; long long ldq;        // roped queries [T][ldq], head h at column h*128
-  bf16* out; long long ldo;            // [T][ldo]
-  const bf16* kcache; const bf16* vcache;  // this layer
-  const int32_t* page_table; int max_pages;
-  const int32_t* cu_seqlens;           // [B+1] token offsets of each sequence in the packed buffers
-  const int32_t* seq_slot;             // [B] row of the page table
-  int nh, nkv;
-  float scale_log2;                    // (1/sqrt(d)) * log2(e)
-};
-
-__global__ void __launch_bounds__(kAttnThreads) attn_prefill_kernel(const AttnPrefillParams p) {
-  TraceScope _ts(TK_ATTN_PREFILL);
-  pdl_launch_dependents();
-  pdl_wait();
-  _ts.mark();
-  extern __shared__ __align__(1024) uint8_t smem[];
-  const int b = blockIdx.z, h = blockIdx.y, qt = blockIdx.x;
-  const int tok0 = p.cu_seqlens[b];
-  const int len = p.cu_seqlens[b + 1] - tok0;
-  const int q0 = qt * 64;
-  if (q0 >= len) return;
-  const int kvh = h / (p.nh / p.nkv);
-  const int slot = p.seq_slot[b];
-  const int32_t* pages = p.page_table + (long long)slot * p.max_pages;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int g = lane >> 2, t = lane & 3;
-  const uint32_t sQ = smem_u32(smem);
-  const uint32_t sK = sQ + kTileBytes;      // 2 buffers
-  const uint32_t sV = sK + 2 * kTileBytes;  // 2 buffers
-  const long long tile_stride = (long long)p.nkv * kPageTokens * kHeadDim;
-  const long long head_off = (long long)kvh * kPageTokens * kHeadDim;
-
-  // Q tile (rows beyond the sequence are zero-filled)
-#pragma unroll
-  for (int it = 0; it < 8; ++it) {
-    const int idx = threadIdx.x + it * kAttnThreads;
-    const int r = idx >> 4, c = idx & 15;
-    const bool valid = (q0 + r) < len;
-    const bf16* src = p.q + (long long)(tok0 + (valid ? q0 + r : 0)) * p.ldq + h * kHeadDim + c * 8;
-    cp_async_16(sQ + swz(r, c), src, valid);
-  }
-  const int ntiles = qt + 1;  // causal: KV tiles 0..qt
-  load_kv_tile(sK, p.kcache + (long long)pages[0] * tile_stride + head_off);
-  load_kv_tile(sV, p.vcache + (long long)pages[0] * tile_stride + head_off);
-  cp_async_commit();
-
-  uint32_t qf[8][4];
-  float o[16][4];
-#pragma unroll
-  for (int i = 0; i < 16; ++i) o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f;
-  float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-  const int wrow = warp * 16;
-
-  for (int j = 0; j < ntiles; ++j) {
-    const int buf = j & 1;
-    if (j + 1 < ntiles) {
-      const long long pg = pages[j + 1];
-      load_kv_tile(sK + (buf ^ 1) * kTileBytes, p.kcache + pg * tile_stride + head_off);
-      load_kv_tile(sV + (buf ^ 1) * kTileBytes, p.vcache + pg * tile_stride + head_off);
-      cp_async_commit();
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncthreads();
-    if (j == 0) {
-#pragma unroll
-      for (int ks = 0; ks < 8; ++ks)
-        ldmatrix_x4(qf[ks], sQ + swz(wrow + (lane & 7) + 8 * ((lane >> 3) & 1), 2 * ks + (lane >> 4)));
-    }
-    float s[8][4];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) s[i][0] = s[i][1] = s[i][2] = s[i][3] = 0.f;
-    const uint32_t sKb = sK + buf * kTileBytes, sVb = sV + buf * kTileBytes;
-#pragma unroll
-    for (int ks = 0; ks < 8; ++ks) {
-#pragma unroll
-      for (int np = 0; np < 4; ++np) {
-        uint32_t bfr[4];
-        ldmatrix_x4(bfr, sKb + swz(16 * np + (lane & 7) + 8 * (lane >> 4), 2 * ks + ((lane >> 3) & 1)));
-        mma_m16n8k16_bf16(s[2 * np], qf[ks], bfr[0], bfr[1]);
-        mma_m16n8k16_bf16(s[2 * np + 1], qf[ks], bfr[2], bfr[3]);
-      }
-    }
-    // scale (log2 domain) + causal mask on the diagonal tile
-    const bool diag = (j == qt);
-    const int qp0 = q0 + wrow + g, qp1 = qp0 + 8;
-    float mx0 = -INFINITY, mx1 = -INFINITY;
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-#pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        const int kp = j * 64 + nt * 8 + 2 * t + e;
-        float v0 = s[nt][e] * p.scale_log2, v1 = s[nt][2 + e] * p.scale_log2;
-        if (diag && kp > qp0) v0 = -INFINITY;
-        if (diag && kp > qp1) v1 = -INFINITY;
-        s[nt][e] = v0;
-        s[nt][2 + e] = v1;
-        mx0 = fmaxf(mx0, v0);
-        mx1 = fmaxf(mx1, v1);
-      }
-    }
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-    const float mn0 = fmaxf(m0, mx0), mn1 = fmaxf(m1, mx1);  // finite: key 0 is never masked
-    const float c0 = exp2f(m0 - mn0), c1 = exp2f(m1 - mn1);
-    m0 = mn0; m1 = mn1;
-    l0 *= c0; l1 *= c1;
-#pragma unroll
-    for (int i = 0; i < 16; ++i) { o[i][0] *= c0; o[i][1] *= c0; o[i][2] *= c1; o[i][3] *= c1; }
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-      s[nt][0] = exp2f(s[nt][0] - mn0); s[nt][1] = exp2f(s[nt][1] - mn0);
-      s[nt][2] = exp2f(s[nt][2] - mn1); s[nt][3] = exp2f(s[nt][3] - mn1);
-      l0 += s[nt][0] + s[nt][1];
-      l1 += s[nt][2] + s[nt][3];
-    }
-#pragma unroll
-    for (int kk = 0; kk < 4; ++kk) {
-      uint32_t a[4];
-      a[0] = pack_bf16x2(s[2 * kk][0], s[2 * kk][1]);
-      a[1] = pack_bf16x2(s[2 * kk][2], s[2 * kk][3]);
-      a[2] = pack_bf16x2(s[2 * kk + 1][0], s[2 * kk + 1][1]);
-      a[3] = pack_bf16x2(s[2 * kk + 1][2], s[2 * kk + 1][3]);
-#pragma unroll
-      for (int dp = 0; dp < 8; ++dp) {
-        uint32_t bfr[4];
-        ldmatrix_x4_trans(bfr, sVb + swz(16 * kk + (lane & 7) + 8 * ((lane >> 3) & 1), 2 * dp + (lane >> 4)));
-        mma_m16n8k16_bf16(o[2 * dp], a, bfr[0], bfr[1]);
-        mma_m16n8k16_bf16(o[2 * dp + 1], a, bfr[2], bfr[3]);
-      }
-    }
-    __syncthreads();
-  }
-  l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-  l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-  const float i0 = 1.f / l0, i1 = 1.f / l1;
-  const int r0 = q0 + wrow + g, r1 = r0 + 8;
-#pragma unroll
-  for (int nt = 0; nt < 16; ++nt) {
-    const int col = h * kHeadDim + nt * 8 + 2 * t;
-    if (r0 < len)
-      *reinterpret_cast<uint32_t*>(p.out + (long long)(tok0 + r0) * p.ldo + col) = pack_bf16x2(o[nt][0] * i0, o[nt][1] * i0);
-    if (r1 < len)
-      *reinterpret_cast<uint32_t*>(p.out + (long long)(tok0 + r1) * p.ldo + col) = pack_bf16x2(o[nt][2] * i1, o[nt][3] * i1);
-  }
-}
-
 struct AttnDecodeParams {
   const bf16* q; long long ldq;        // [B][ldq] roped queries of the current token
   bf16* out; long long ldo;            // [B][ldo]
@@ -205,9 +52,9 @@ struct AttnDecodeParams {
   const float* qkv_partial; int qkv_splits; long long qkv_split_stride; long long ld_qkv_partial;
   const bf16* cos_tab; const bf16* sin_tab;
   bf16* kcache_w; bf16* vcache_w;
-  // splits > 1: per-(sequence, kv head) arrival counters (zero between launches).  When set, the LAST split CTA to
-  // arrive merges the partials itself (in split order: deterministic) and no attn_combine_kernel follows — one kernel
-  // boundary less on the tensor-parallel decode path, where few (sequence, kv head) pairs per GPU force the split.
+  // splits > 1: per-(sequence, kv head) arrival counters (zero between launches; required).  The LAST split CTA to
+  // arrive merges the partials itself (in split order: deterministic) — no separate combine kernel on the
+  // tensor-parallel decode path, where few (sequence, kv head) pairs per GPU force the split.
   int* split_counter;
 };
 
@@ -490,33 +337,6 @@ __global__ void __launch_bounds__(kAttnThreads) attn_decode_kernel(const AttnDec
     }
   }
   if (p.splits > 1 && p.split_counter) attn_decode_arrive_and_merge(p, bh, b, kvh);
-}
-
-// one CTA (128 threads) per (batch row, query head)
-__global__ void __launch_bounds__(128)
-attn_combine_kernel(const float* __restrict__ part_o, const float* __restrict__ part_ml, bf16* __restrict__ out,
-                    long long ldo, int nkv, int G, int splits) {
-  TraceScope _ts(TK_ATTN_COMBINE);
-  pdl_launch_dependents();
-  pdl_wait();
-  _ts.mark();
-  const int bhq = blockIdx.x;            // b * nh + head
-  const int nh = nkv * G;
-  const int b = bhq / nh, head = bhq - b * nh;
-  const int kvh = head / G, r = head - kvh * G;
-  const long long base = ((long long)(b * nkv + kvh) * splits) * G;
-  float M = -INFINITY;
-  for (int s = 0; s < splits; ++s) M = fmaxf(M, part_ml[(base + (long long)s * G + r) * 2]);
-  float L = 0.f, acc = 0.f;
-  const int d = threadIdx.x;
-  for (int s = 0; s < splits; ++s) {
-    const long long row = base + (long long)s * G + r;
-    const float ms = part_ml[row * 2];
-    const float f = (ms == -INFINITY) ? 0.f : exp2f(ms - M);
-    L += part_ml[row * 2 + 1] * f;
-    acc += part_o[row * kHeadDim + d] * f;
-  }
-  out[(long long)b * ldo + head * kHeadDim + d] = __float2bfloat16_rn(acc / L);
 }
 
 }  // namespace b200

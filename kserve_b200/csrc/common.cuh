@@ -83,7 +83,7 @@ struct TraceRec { unsigned long long t0, t1, tmid; int kind, block; };
 __device__ TraceRec* g_trace_buf = nullptr;
 __device__ unsigned int g_trace_cap = 0;
 __device__ unsigned int g_trace_cnt = 0;
-enum TraceKind : int { TK_GEMM = 1, TK_RMSNORM = 2, TK_ROPE = 3, TK_ATTN_DECODE = 4, TK_ATTN_COMBINE = 5, TK_ARGMAX = 6,
+enum TraceKind : int { TK_GEMM = 1, TK_RMSNORM = 2, TK_ROPE = 3, TK_ATTN_DECODE = 4, TK_ARGMAX = 6,
                        TK_STEP = 7, TK_EMBED = 8, TK_ATTN_PREFILL = 9, TK_OTHER = 10 };
 __device__ __forceinline__ unsigned long long global_timer() {
   unsigned long long t;
@@ -195,13 +195,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
       " [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(smem_u32(smem_dst)),
       "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c_inner), "r"(c_outer), "l"(hint)
       : "memory");
-}
-// Asynchronous prefetch of a 2D tile into L2 only (no shared memory): used to pull the next weight slab towards
-// the SMs while the kernel is still waiting for its predecessor.
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* map, int c_inner, int c_outer) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(map)),
-               "r"(c_inner), "r"(c_outer)
-               : "memory");
 }
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");

@@ -215,14 +215,7 @@ struct b200_engine {
   std::vector<char> cb_slot_sampling;    // slot uses the processed-score path
   int cb_sampling_slots = 0;
   int32_t* d_kv_off = nullptr;           // [80] tokens of each prefill row's sequence that are already cached
-  // weight-stream L2 prefetch (prefetch.cuh): the step's weight-streaming GEMMs in launch order, per graph key
-  PfCtx pf;
-  std::unordered_map<int, std::vector<PfGemm>> pf_tables;
-  const std::vector<PfGemm>* pf_cur = nullptr;   // table of the step being captured (nullptr: no prefetch launches)
-  cudaEvent_t ev_pf_fork = nullptr, ev_pf_join = nullptr;
-  bool faulted = false;                          // a cross-GPU / cross-CTA wait timed out (common.cuh: g_fault_code)
-  int pf_cap_kb = 16;                            // k-block tiles (16 KB each) prefetched per CTA of the next GEMM
-  bool pf_forked = false;
+  bool faulted = false;                  // a cross-GPU / cross-CTA wait timed out (common.cuh: g_fault_code)
 };
 
 namespace b200 {
@@ -232,32 +225,11 @@ static int pick_block_n(int B) { return B <= 16 ? 16 : (B <= 32 ? 32 : 64); }
 
 // peer-memory all-reduce + residual + RMSNorm of the decode step: one-shot LL up to 4 ranks, two-shot (reduce-scatter +
 // all-gather, 4x less NVLink traffic) at 8 ranks.  Measured r02: TP = 8 decode 2.64 -> 2.20 ms/step with two-shot; at TP = 4
-// two-shot is slower (2.57 vs 2.46 ms/step: one more NVLink hop for only 2x less traffic).  B200_AR_TWO_SHOT_MIN_TP moves the switch.
+// two-shot is slower (2.57 vs 2.46 ms/step: one more NVLink hop for only 2x less traffic).
 typedef void (*ArKernel)(const P2P, bf16*, const bf16*, bf16*, float, const float*, int, long long, long long, const bf16*, int, int);
 static ArKernel ar_kernel(const b200_engine* e) {
-  static const int min_tp = getenv("B200_AR_TWO_SHOT_MIN_TP") ? atoi(getenv("B200_AR_TWO_SHOT_MIN_TP")) : 8;
-  return (e->cfg.tp_size >= min_tp && (e->H / e->cfg.tp_size) % 8 == 0) ? allreduce2_norm_kernel : allreduce_norm_kernel;
-}
-
-// every GEMM of the engine goes through here so that the decode step's weight-streaming launches join the
-// prefetcher's table (launch.cuh: PfCtx) without threading the context through each call site
-static int launch_gemm(b200_engine* e, GemmArgs& a, int sms, cudaStream_t s) {
-  a.pf = &e->pf;
-  if (e->pf_cur && e->pf.active && pf_eligible(a) && s == e->stream) {
-    // capture: beside GEMM i (it starts when its predecessor in the chain has completed) prefetch the head of GEMM i+1's
-    // weight stream; after the step's last GEMM (LM head) that is the first GEMM of the next step (L2 survives the launch)
-    const std::vector<PfGemm>& tab = *e->pf_cur;
-    const int i = e->pf.count;
-    if (i < (int)tab.size()) {
-      const PfGemm& nxt = tab[(i + 1) % tab.size()];
-      B200_CUDA_OK(cudaEventRecord(e->ev_pf_fork, s));
-      B200_CUDA_OK(cudaStreamWaitEvent(e->stream2, e->ev_pf_fork, 0));
-      weight_prefetch_kernel<<<nxt.grid, 32, 0, e->stream2>>>(nxt, e->pf_cap_kb);
-      B200_CUDA_OK(cudaGetLastError());
-      e->pf_forked = true;
-    }
-  }
-  return launch_gemm(e->tmaps, a, sms, s);
+  constexpr int kTwoShotMinTp = 8;
+  return (e->cfg.tp_size >= kTwoShotMinTp && (e->H / e->cfg.tp_size) % 8 == 0) ? allreduce2_norm_kernel : allreduce_norm_kernel;
 }
 
 static int pick_splits(const b200_engine* e, int n_out, int K) {
@@ -274,11 +246,11 @@ static int pick_splits(const b200_engine* e, int n_out, int K) {
 static int allreduce_bf16(b200_engine* e, bf16* buf, size_t count, cudaStream_t s) {
   if (e->cfg.tp_size == 1) return 0;
   static const bool force_nccl = getenv("B200_PREFILL_OWN_AR") == nullptr;
-  static const int ar_ctas = getenv("B200_PREFILL_AR_CTAS") ? atoi(getenv("B200_PREFILL_AR_CTAS")) : 64;
+  constexpr int kArCtas = 64;
   if (e->p2p_ready && !force_nccl && buf >= e->ybuf && buf + count <= e->ybuf + (size_t)e->cap_T * e->H && count % 8 == 0) {
     const int lane = (s == e->stream2) ? 1 : 0;
     const int epoch = ++e->big_epoch[lane];
-    allreduce_big_kernel<<<ar_ctas, 256, 0, s>>>(e->p2p, (long long)e->p2p.lay.total, (long long)(buf - e->ybuf), (long long)count,
+    allreduce_big_kernel<<<kArCtas, 256, 0, s>>>(e->p2p, (long long)e->p2p.lay.total, (long long)(buf - e->ybuf), (long long)count,
                                                  epoch, lane, e->big_cnt + lane);
     B200_CUDA_OK(cudaGetLastError());
     e->launches++;
@@ -306,20 +278,15 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
   // half's GEMMs / attention own the SMs (SURVEY.md §8e "prefill ... overlap by token-chunking").
   struct View { long long r0; int T, b0, B; cudaStream_t s; };
   View views[2] = {{0, T_all, 0, B_all, e->stream}, {0, 0, 0, 0, e->stream2}};
-  int nv = 1, gsms = e->num_sms;   // SMs the GEMM grids are sized for
-  static const bool mb_off = getenv("B200_NO_PREFILL_OVERLAP") != nullptr;
+  int nv = 1;
   static const int mb_min_t = getenv("B200_PREFILL_OVERLAP_MIN_T") ? atoi(getenv("B200_PREFILL_OVERLAP_MIN_T")) : 2048;
-  if (!decode && tp && e->E == 0 && B_all >= 2 && T_all >= mb_min_t && !mb_off) {
+  if (!decode && tp && e->E == 0 && B_all >= 2 && T_all >= mb_min_t) {
     const int b0 = B_all / 2;
     long long r0 = 0;
     for (int b = 0; b < b0; ++b) r0 += e->st.lens[b];
     views[0] = View{0, (int)r0, 0, b0, e->stream};
     views[1] = View{r0, (int)(T_all - r0), b0, B_all - b0, e->stream2};
     nv = 2;
-    // leave a few SMs to the collective: the persistent GEMM grids would otherwise wait for them tile-round after tile-round
-    static const int reserve = getenv("B200_PREFILL_RESERVE_SMS") ? atoi(getenv("B200_PREFILL_RESERVE_SMS")) : 0;
-    static const int mult = getenv("B200_PREFILL_GRID_MULT") ? atoi(getenv("B200_PREFILL_GRID_MULT")) : 1;
-    gsms = std::max(2, e->num_sms - reserve) * std::max(1, mult);
     B200_CUDA_OK(cudaEventRecord(e->ev_fork, e->stream));
     B200_CUDA_OK(cudaStreamWaitEvent(e->stream2, e->ev_fork, 0));
   }
@@ -342,7 +309,6 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
     bf16* vc = e->vcache + (long long)l * e->layer_stride;
     // ---- QKV projection
     RopeKvParams rp{};
-    bool fused_rope = false;
     rp.ld = e->qkv_cols;
     if (decode) {
       // uniform split-K with fp32 partials: the consumer kernel (attention prologue / rmsnorm) reduces them in
@@ -351,7 +317,7 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
       GemmArgs a{w.wqkv, e->qkv_cols, e->xn, e->cap_T, e->qkv_cols, B, H, sp > 1 ? EPI_T_PARTIAL : EPI_T_STORE, bn, sp,
                  sp > 1 ? (void*)e->ws : (void*)e->qkv, nullptr, e->qkv_cols, (long long)B * e->qkv_cols, 0, true};
       a.sk_ws = e->sk_ws; a.sk_flags = e->sk_flags; a.sk_tiles = e->sk_tiles; a.sk_ws_floats = e->sk_ws_floats;
-      if ((rc = launch_gemm(e, a, e->num_sms, s))) return rc;
+      if ((rc = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc;
       if (sp > 1) { rp.partial = e->ws; rp.splits = sp; rp.split_stride = (long long)B * e->qkv_cols; rp.ld_partial = e->qkv_cols; }
       rp.qkv = e->qkv;
       rp.q_out = e->qdec; rp.ldq = e->nh * kHeadDim;
@@ -362,23 +328,14 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
       rp.tok_seq = e->d_tok_seq + r0; rp.tok_pos = e->d_tok_pos + r0;
       rp.kcache = kc; rp.vcache = vc; rp.page_table = e->d_page_table; rp.max_pages = e->max_pages;
       rp.cos_tab = e->cos_tab; rp.sin_tab = e->sin_tab; rp.nh = e->nh; rp.nkv = e->nkv;
-      // RoPE + KV append in the QKV GEMM's epilogue (the separate rope_kv_kernel pass re-read and re-wrote 750 MB per layer
-      // at 0.37 of the HBM peak); B200_NO_ROPE_FUSION=1 / B200_NO_2CTA=1 restore the two-kernel path
-      static const bool rope_fused = getenv("B200_NO_ROPE_FUSION") == nullptr && getenv("B200_NO_2CTA") == nullptr;
-      fused_rope = rope_fused;
-      GemmArgs a{e->xn + r0 * H, e->cap_T - (int)r0, w.wqkv, e->qkv_cols, T, e->qkv_cols, H, fused_rope ? EPI_ROPE_KV : EPI_STORE, 256, 1,
+      // RoPE + KV append in the QKV GEMM's epilogue (a separate rope_kv_kernel pass re-read and re-wrote 750 MB per layer
+      // at 0.37 of the HBM peak); decode fuses them into attn_decode_kernel instead
+      GemmArgs a{e->xn + r0 * H, e->cap_T - (int)r0, w.wqkv, e->qkv_cols, T, e->qkv_cols, H, EPI_ROPE_KV, 256, 1,
                  e->qkv + r0 * e->qkv_cols, nullptr, e->qkv_cols, 0, 0, false};
       a.rope = &rp;
-      if ((rc = launch_gemm(e, a, gsms, s))) return rc;
+      if ((rc = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc;
     }
-    rp.kcache = kc; rp.vcache = vc; rp.page_table = e->d_page_table; rp.max_pages = e->max_pages;
-    rp.cos_tab = e->cos_tab; rp.sin_tab = e->sin_tab; rp.nh = e->nh; rp.nkv = e->nkv;
     e->launches++;
-    if (!decode && !fused_rope) {   // decode: RoPE + KV append are fused into attn_decode_kernel
-      rp.T = T; rp.tokens_per_cta = 1;   // (4 tokens per CTA measured SLOWER: 446 vs 312 us per launch, r02 ncu)
-      B200_CUDA_OK(launch_k(rope_kv_kernel, dim3((T + rp.tokens_per_cta - 1) / rp.tokens_per_cta), dim3(512), 0, s, rp));
-      e->launches++;
-    }
     // ---- attention
     if (decode) {
       AttnDecodeParams ap{};
@@ -389,32 +346,19 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
       // when there are fewer CTAs than SMs
       const int ctas = B * e->nkv;
       ap.splits = ctas >= e->num_sms ? 1 : std::max(1, std::min((e->num_sms + ctas - 1) / ctas, 8));
-      static const int force_splits = getenv("B200_ATTN_SPLITS") ? atoi(getenv("B200_ATTN_SPLITS")) : 0;   // (A/B)
-      if (force_splits > 0) ap.splits = std::min(force_splits, 8);
       ap.part_o = e->part_o; ap.part_ml = e->part_ml; ap.scale_log2 = scale_log2;
       ap.fuse_rope = 1; ap.qkv = rp.qkv; ap.ld_qkv = rp.ld; ap.qkv_partial = rp.partial; ap.qkv_splits = rp.splits;
       ap.qkv_split_stride = rp.split_stride; ap.ld_qkv_partial = rp.ld_partial; ap.cos_tab = e->cos_tab; ap.sin_tab = e->sin_tab;
       ap.kcache_w = kc; ap.vcache_w = vc;
-      static const bool fold = getenv("B200_ATTN_COMBINE_KERNEL") == nullptr;   // =1: separate attn_combine_kernel (A/B)
-      ap.split_counter = fold ? e->attn_split_cnt : nullptr;
+      ap.split_counter = e->attn_split_cnt;
       if ((rc = launch_attn_decode(ap, B, s))) return rc;
-      e->launches += (ap.splits > 1 && !ap.split_counter) ? 2 : 1;
+      e->launches++;
     } else {
-      AttnPrefillParams ap{};
-      ap.q = e->qkv; ap.ldq = e->qkv_cols; ap.out = e->attn; ap.ldo = e->nh * kHeadDim;
-      ap.kcache = kc; ap.vcache = vc; ap.page_table = e->d_page_table; ap.max_pages = e->max_pages;
-      ap.cu_seqlens = e->d_cu + vw.b0; ap.seq_slot = e->d_seq_slot + vw.b0; ap.nh = e->nh; ap.nkv = e->nkv; ap.scale_log2 = scale_log2;
-      static const bool attn_mma = getenv("B200_ATTN_MMA") != nullptr;   // legacy mma.sync kernel for A/B runs
-      if (attn_mma) {
-        B200_REQUIRE(kv_off == nullptr, "chunked prefill / prefix reuse needs the tcgen05 attention kernel (unset B200_ATTN_MMA)");
-        if ((rc = launch_attn_prefill(ap, B, max_len, s))) return rc;
-      } else {
-        AttnTcParams tp_{};
-        tp_.out = e->attn; tp_.ldo = e->nh * kHeadDim; tp_.page_table = e->d_page_table; tp_.max_pages = e->max_pages;
-        tp_.cu_seqlens = e->d_cu + vw.b0; tp_.seq_slot = e->d_seq_slot + vw.b0; tp_.nh = e->nh; tp_.nkv = e->nkv; tp_.scale_log2 = scale_log2;
-        tp_.kv_off = kv_off ? kv_off + vw.b0 : nullptr;
-        if ((rc = launch_attn_prefill_tc(e->tmaps, e->qkv, e->cap_T, e->qkv_cols, kc, vc, e->num_pages, tp_, B, max_len, s))) return rc;
-      }
+      AttnTcParams tp_{};
+      tp_.out = e->attn; tp_.ldo = e->nh * kHeadDim; tp_.page_table = e->d_page_table; tp_.max_pages = e->max_pages;
+      tp_.cu_seqlens = e->d_cu + vw.b0; tp_.seq_slot = e->d_seq_slot + vw.b0; tp_.nh = e->nh; tp_.nkv = e->nkv; tp_.scale_log2 = scale_log2;
+      tp_.kv_off = kv_off ? kv_off + vw.b0 : nullptr;
+      if ((rc = launch_attn_prefill_tc(e->tmaps, e->qkv, e->cap_T, e->qkv_cols, kc, vc, e->num_pages, tp_, B, max_len, s))) return rc;
       e->launches++;
     }
     // ---- row-parallel projections (o_proj, down_proj) followed by residual add + next RMSNorm
@@ -424,7 +368,7 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
         const int sp = pick_splits(e, H, K);
         if (sp > 1) {
           GemmArgs a{wmat, H, act, e->cap_T, H, B, K, EPI_T_PARTIAL, bn, sp, e->ws, nullptr, H, (long long)B * H, 0, true};
-          if ((rc2 = launch_gemm(e, a, e->num_sms, s))) return rc2;
+          if ((rc2 = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc2;
           e->launches++;
           if (!tp) {
             if ((rc2 = launch_rmsnorm(1, e->x, next_norm, e->xn, T, H, eps, e->ws, sp, (long long)B * H, H, nullptr, s))) return rc2;
@@ -443,7 +387,7 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
         } else {
           GemmArgs a{wmat, H, act, e->cap_T, H, B, K, EPI_T_STORE, bn, 1, e->ybuf, nullptr, H, 0, 0, true};
           a.sk_ws = e->sk_ws; a.sk_flags = e->sk_flags; a.sk_tiles = e->sk_tiles; a.sk_ws_floats = e->sk_ws_floats;
-          if ((rc2 = launch_gemm(e, a, e->num_sms, s))) return rc2;
+          if ((rc2 = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc2;
           e->launches++;
           if (tp && e->p2p_ready) {
             B200_CUDA_OK(launch_k(ar_kernel(e), dim3(T), dim3(kNormThreads), (size_t)(H + 32) * sizeof(float), s, e->p2p,
@@ -456,13 +400,13 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
       } else {
         if (!tp) {
           GemmArgs a{act, e->cap_T, wmat, H, T, H, K, EPI_STORE_RES, 256, 1, e->x, e->x, H, 0, 0, false};   // (r0 == 0: one GPU)
-          if ((rc2 = launch_gemm(e, a, gsms, s))) return rc2;
+          if ((rc2 = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc2;
           if ((rc2 = launch_rmsnorm(0, e->x, next_norm, e->xn, T, H, eps, nullptr, 0, 0, 0, nullptr, s))) return rc2;
           e->launches += 2;
           return 0;
         }
         GemmArgs a{act + r0 * K, e->cap_T - (int)r0, wmat, H, T, H, K, EPI_STORE, 256, 1, e->ybuf + r0 * H, nullptr, H, 0, 0, false};
-        if ((rc2 = launch_gemm(e, a, gsms, s))) return rc2;
+        if ((rc2 = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc2;
         e->launches++;
       }
       if ((rc2 = allreduce_bf16(e, e->ybuf + r0 * H, (size_t)T * H, s))) return rc2;
@@ -488,46 +432,31 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
         e->launches += 3;
       }
       // decode: ONE grouped launch per projection over all experts (E * tiles fill the SMs; the weights of experts
-      // without tokens are skipped).  B200_MOE_PER_EXPERT=1 restores one launch per expert (A/B).
-      static const bool per_expert = getenv("B200_MOE_PER_EXPERT") != nullptr;
-      const bool grouped = decode && !per_expert;
-      const int dsp = (decode && !grouped) ? pick_splits(e, H, e->I) : 1;
-      if (grouped) {
+      // without tokens are skipped); prefill: one 2-CTA launch per expert, bounded by the expert's token count
+      if (decode) {
         GemmArgs a{w.wgu_e, e->E * 2 * e->I, e->xg, e->g_rows, 2 * e->I, B, H, EPI_T_SWIGLU, bn, 1, e->hg, nullptr, e->I, 0, e->I, true};
         a.n_rt = e->e_count; a.row_off = e->e_off; a.groups = e->E;
-        if ((rc = launch_gemm(e, a, e->num_sms, s))) return rc;
+        if ((rc = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc;
         GemmArgs d{w.wdown_e, e->E * H, e->hg, e->g_rows, H, B, e->I, EPI_T_STORE, bn, 1, e->yg, nullptr, H, 0, 0, true};
         d.n_rt = e->e_count; d.row_off = e->e_off; d.groups = e->E;
-        if ((rc = launch_gemm(e, d, e->num_sms, s))) return rc;
+        if ((rc = launch_gemm(e->tmaps, d, e->num_sms, s))) return rc;
         e->launches += 2;
       }
-      for (int x = 0; x < e->E && !grouped; ++x) {
+      for (int x = 0; x < e->E && !decode; ++x) {
         const bf16* wgu = w.wgu_e + (long long)x * 2 * e->I * H;
         const bf16* wdn = w.wdown_e + (long long)x * H * e->I;
-        if (decode) {
-          GemmArgs a{wgu, 2 * e->I, e->xg, e->g_rows, 2 * e->I, B, H, EPI_T_SWIGLU, bn, 1, e->hg, nullptr, e->I, 0, e->I, true};
-          a.sk_ws = e->sk_ws; a.sk_flags = e->sk_flags; a.sk_tiles = e->sk_tiles; a.sk_ws_floats = e->sk_ws_floats;
-          a.n_rt = e->e_count + x; a.row_off = e->e_off + x;
-          if ((rc = launch_gemm(e, a, e->num_sms, s))) return rc;
-          GemmArgs d{wdn, H, e->hg, e->g_rows, H, B, e->I, dsp > 1 ? EPI_T_PARTIAL : EPI_T_STORE, bn, dsp,
-                     dsp > 1 ? (void*)(e->ws + (size_t)x * dsp * B * H) : (void*)e->yg, nullptr, H, (long long)B * H, 0, true};
-          d.n_rt = e->e_count + x; d.row_off = e->e_off + x;
-          if ((rc = launch_gemm(e, d, e->num_sms, s))) return rc;
-        } else {
-          GemmArgs a{e->xg, e->g_rows, wgu, 2 * e->I, T, 2 * e->I, H, EPI_SWIGLU, 256, 1, e->hg, nullptr, e->I, 0, e->I, false};
-          a.m_rt = e->e_count + x; a.row_off = e->e_off + x;
-          if ((rc = launch_gemm(e, a, gsms, s))) return rc;
-          GemmArgs d{e->hg, e->g_rows, wdn, H, T, H, e->I, EPI_STORE, 256, 1, e->yg, nullptr, H, 0, 0, false};
-          d.m_rt = e->e_count + x; d.row_off = e->e_off + x;
-          if ((rc = launch_gemm(e, d, gsms, s))) return rc;
-        }
+        GemmArgs a{e->xg, e->g_rows, wgu, 2 * e->I, T, 2 * e->I, H, EPI_SWIGLU, 256, 1, e->hg, nullptr, e->I, 0, e->I, false};
+        a.m_rt = e->e_count + x; a.row_off = e->e_off + x;
+        if ((rc = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc;
+        GemmArgs d{e->hg, e->g_rows, wdn, H, T, H, e->I, EPI_STORE, 256, 1, e->yg, nullptr, H, 0, 0, false};
+        d.m_rt = e->e_count + x; d.row_off = e->e_off + x;
+        if ((rc = launch_gemm(e->tmaps, d, e->num_sms, s))) return rc;
         e->launches += 2;
       }
       MoeCombineParams cp{};
       cp.x = e->x; cp.w = next_norm; cp.xn = e->xn; cp.H = H; cp.eps = eps;
-      cp.tok_expert = e->tok_expert; cp.tok_weight = e->tok_weight; cp.tok_row = e->tok_row; cp.off = e->e_off;
+      cp.tok_expert = e->tok_expert; cp.tok_weight = e->tok_weight; cp.tok_row = e->tok_row;
       cp.yg = e->yg;
-      if (decode && dsp > 1) { cp.part = e->ws; cp.splits = dsp; cp.expert_stride = (long long)dsp * B * H; cp.split_stride = (long long)B * H; }
       cp.ysum = tp ? e->ybuf : nullptr;
       B200_CUDA_OK(launch_k(moe_combine_norm_kernel, dim3(T), dim3(kNormThreads), (size_t)(H + 32) * sizeof(float), s, cp));
       e->launches++;
@@ -546,23 +475,22 @@ static int forward_layers(b200_engine* e, int T_all, int B_all, int max_len, boo
     // ---- gate/up projection with the SwiGLU fused into the epilogue
     if (decode) {
       const int gu_tiles = (2 * e->I + kGemmBlockM - 1) / kGemmBlockM;
-      static const bool gu_sk = getenv("B200_GU_STREAMK") != nullptr;
-      const int gsp = (gu_sk || gu_tiles * 4 >= e->num_sms * 3) ? 1 : pick_splits(e, 2 * e->I, H);
+      const int gsp = gu_tiles * 4 >= e->num_sms * 3 ? 1 : pick_splits(e, 2 * e->I, H);
       if (gsp > 1) {   // few tiles per GPU (tensor parallel): split-K partials + a reducing SwiGLU kernel
         GemmArgs a{w.wgu, 2 * e->I, e->xn, e->cap_T, 2 * e->I, B, H, EPI_T_PARTIAL, bn, gsp, e->ws, nullptr, 2 * e->I,
                    (long long)B * 2 * e->I, 0, true};
-        if ((rc = launch_gemm(e, a, e->num_sms, s))) return rc;
+        if ((rc = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc;
         B200_CUDA_OK(launch_k(swiglu_reduce_kernel, dim3(B), dim3(512), 0, s, (const float*)e->ws, gsp, (long long)B * 2 * e->I,
                               (long long)2 * e->I, e->hbuf, e->I));
         e->launches++;
       } else {
         GemmArgs a{w.wgu, 2 * e->I, e->xn, e->cap_T, 2 * e->I, B, H, EPI_T_SWIGLU, bn, 1, e->hbuf, nullptr, e->I, 0, e->I, true};
         a.sk_ws = e->sk_ws; a.sk_flags = e->sk_flags; a.sk_tiles = e->sk_tiles; a.sk_ws_floats = e->sk_ws_floats;
-        if ((rc = launch_gemm(e, a, e->num_sms, s))) return rc;
+        if ((rc = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc;
       }
     } else {
       GemmArgs a{e->xn + r0 * H, e->cap_T - (int)r0, w.wgu, 2 * e->I, T, 2 * e->I, H, EPI_SWIGLU, 256, 1, e->hbuf + r0 * e->I, nullptr, e->I, 0, e->I, false};
-      if ((rc = launch_gemm(e, a, gsms, s))) return rc;
+      if ((rc = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc;
     }
     e->launches++;
     if ((rc = row_parallel(e->hbuf, e->I, w.wdown, next_norm))) return rc;
@@ -582,7 +510,7 @@ static int head_and_step(b200_engine* e, const bf16* rows_xn, int rows_cap, int 
   GemmArgs a{e->lm_head, e->Vl, rows_xn, rows_cap, e->Vl, B, e->H, EPI_T_STORE, pick_block_n(B), 1,
              e->logits, nullptr, e->Vl, 0, 0, true};
   a.sk_ws = e->sk_ws; a.sk_flags = e->sk_flags; a.sk_tiles = e->sk_tiles; a.sk_ws_floats = e->sk_ws_floats;
-  if ((rc = launch_gemm(e, a, e->num_sms, s))) return rc;
+  if ((rc = launch_gemm(e->tmaps, a, e->num_sms, s))) return rc;
   const int use_p2p = (e->cfg.tp_size > 1 && e->p2p_ready) ? 1 : 0;
   // one GPU: 16 CTAs per row scan slices of the 128k-entry row (a single CTA per row took 65 us of the 4.3 ms step)
   const int chunks = (e->cfg.tp_size == 1 && e->Vl >= 16384) ? 16 : 1;
@@ -650,38 +578,18 @@ static int decode_step_enqueue(b200_engine* e) {
 }
 
 // One decode step through a CUDA graph captured once per key.  The first call for a key runs the step eagerly (tensor
-// maps / function attributes are created outside of capture, and the weight-stream prefetcher's table is recorded), the
-// second captures it: the main chain (programmatic dependent launches) plus, on a forked branch, the prefetch kernel
-// that walks the step's weight-streaming GEMMs ahead of the chain (prefetch.cuh).
+// maps / function attributes are created outside of capture), the second captures it: one chain of programmatic
+// dependent launches.
 template <class Enqueue>
 static int graph_step(b200_engine* e, int key, Enqueue&& enqueue) {
-  // opt-in (B200_PREFETCHER=1): measured r02 (profiles/r02_prefetch_timelines.md) — the head prefetch does not shorten the
-  // step: each GEMM's post-wait time is a latency chain (B tiles -> MMA -> second ring fill -> epilogue), not HBM time,
-  // and the extra requests compete with the kernels that are streaming
-  static const bool pf_on = getenv("B200_PREFETCHER") != nullptr;
   auto it = e->graphs.find(key);
   if (it == e->graphs.end()) {
     const int before = e->launches;
-    e->pf.active = pf_on; e->pf.recording = pf_on; e->pf.count = 0; e->pf.table.clear(); e->pf_cur = nullptr;
     int rc = enqueue();
-    e->pf.recording = false;
-    if (rc) { e->pf.active = false; return rc; }
+    if (rc) return rc;
     const int per_step = e->launches - before;
-    const int n_pf = (int)e->pf.table.size();
-    if (pf_on && n_pf > 1) {
-      e->pf_tables[key] = e->pf.table;
-      e->pf_cur = &e->pf_tables[key];
-    }
     B200_CUDA_OK(cudaStreamBeginCapture(e->stream, cudaStreamCaptureModeThreadLocal));
-    e->pf.count = 0; e->pf_forked = false;
     rc = enqueue();
-    if (rc == 0 && e->pf_cur && e->pf.count != n_pf) { set_last_error("prefetch table does not match the captured step"); rc = -6; }
-    if (e->pf_forked) {   // join the prefetch branch (a capture must end with every forked stream merged back)
-      cudaEventRecord(e->ev_pf_join, e->stream2);
-      cudaStreamWaitEvent(e->stream, e->ev_pf_join, 0);
-    }
-    const int n_forks = e->pf_cur ? n_pf : 0;
-    e->pf.active = false; e->pf_cur = nullptr;
     cudaGraph_t g = nullptr;
     cudaError_t ce = cudaStreamEndCapture(e->stream, &g);
     e->launches -= per_step;  // the captured enqueue did not execute
@@ -691,7 +599,7 @@ static int graph_step(b200_engine* e, int key, Enqueue&& enqueue) {
     B200_CUDA_OK(cudaGraphInstantiate(&ge, g, 0));
     cudaGraphDestroy(g);
     e->graphs[key] = ge;
-    e->graph_nodes[key] = per_step + n_forks;
+    e->graph_nodes[key] = per_step;
     return 0;  // the eager step above already advanced the sequences by one token
   }
   B200_CUDA_OK(cudaGraphLaunch(it->second, e->stream));
@@ -1274,9 +1182,6 @@ int b200_engine_create(const b200_model_config_t* c, const void* nccl_id, b200_e
   B200_CUDA_OK(cudaStreamCreateWithFlags(&e->stream2, cudaStreamNonBlocking));
   B200_CUDA_OK(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
   B200_CUDA_OK(cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming));
-  B200_CUDA_OK(cudaEventCreateWithFlags(&e->ev_pf_fork, cudaEventDisableTiming));
-  B200_CUDA_OK(cudaEventCreateWithFlags(&e->ev_pf_join, cudaEventDisableTiming));
-  if (getenv("B200_PF_CAP_KB")) e->pf_cap_kb = std::max(1, atoi(getenv("B200_PF_CAP_KB")));
   if (getenv("B200_WAIT_TIMEOUT_MS")) {   // bound of the device-side waits (default 5 s), see common.cuh
     const unsigned long long ns = 1000000ull * (unsigned long long)std::max(1, atoi(getenv("B200_WAIT_TIMEOUT_MS")));
     B200_CUDA_OK(cudaMemcpyToSymbol(g_wait_timeout_ns, &ns, sizeof(ns)));
@@ -1354,7 +1259,6 @@ int b200_engine_create(const b200_model_config_t* c, const void* nccl_id, b200_e
   B200_CUDA_OK(cudaMemset(e->xl, 0, RC * H * 2));
   e->ws_elems = (size_t)16 * RC * std::max(std::max(e->qkv_cols, e->H), 2 * e->I);
   if (e->E) {
-    e->ws_elems = std::max(e->ws_elems, (size_t)e->E * 16 * RC * e->H);
     e->g_rows = 2 * e->cap_T + 8 * e->E + 256;
     if ((rc = dmalloc(&e->tok_expert, (size_t)2 * T))) return rc;
     if ((rc = dmalloc(&e->tok_row, (size_t)2 * T))) return rc;
@@ -1446,8 +1350,6 @@ int b200_engine_destroy(b200_engine_t* e) {
   cudaSetDevice(e->cfg.device);
   cudaDeviceSynchronize();
   for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second);
-  if (e->ev_pf_fork) cudaEventDestroy(e->ev_pf_fork);
-  if (e->ev_pf_join) cudaEventDestroy(e->ev_pf_join);
   if (e->comm) Nccl::get().CommDestroy(e->comm);
   for (int r = 0; r < kMaxTp; ++r) if (e->ar_peer_map[r]) cudaIpcCloseMemHandle(e->ar_peer_map[r]);
   if (e->ar_local) cudaFree(e->ar_local);
@@ -2164,16 +2066,6 @@ int b200_op_rmsnorm(void* x, const void* w, void* xn, int rows, int H, float eps
                         (const bf16*)y, (cudaStream_t)stream);
 }
 
-int b200_op_attn_prefill(const void* q, int64_t ldq, void* out, int64_t ldo, const void* kcache, const void* vcache,
-                         const int32_t* page_table, int max_pages, const int32_t* cu_seqlens, const int32_t* seq_slot,
-                         int B, int max_len, int nh, int nkv, void* stream) {
-  AttnPrefillParams p{};
-  p.q = (const bf16*)q; p.ldq = ldq; p.out = (bf16*)out; p.ldo = ldo; p.kcache = (const bf16*)kcache; p.vcache = (const bf16*)vcache;
-  p.page_table = page_table; p.max_pages = max_pages; p.cu_seqlens = cu_seqlens; p.seq_slot = seq_slot; p.nh = nh; p.nkv = nkv;
-  p.scale_log2 = (1.0f / sqrtf((float)kHeadDim)) * 1.4426950408889634f;
-  return launch_attn_prefill(p, B, max_len, (cudaStream_t)stream);
-}
-
 int b200_op_attn_prefill_tc(const void* q, int64_t ldq, int q_rows, void* out, int64_t ldo, const void* kcache,
                             const void* vcache, int num_pages, const int32_t* page_table, int max_pages,
                             const int32_t* cu_seqlens, const int32_t* seq_slot, int B, int max_len, int nh, int nkv,
@@ -2194,6 +2086,16 @@ int b200_op_attn_decode(const void* q, int64_t ldq, void* out, int64_t ldo, cons
   p.page_table = page_table; p.max_pages = max_pages; p.seq_slot = seq_slot; p.tok_pos = tok_pos; p.nh = nh; p.nkv = nkv;
   p.G = nh / nkv; p.splits = splits; p.part_o = part_o; p.part_ml = part_ml;
   p.scale_log2 = (1.0f / sqrtf((float)kHeadDim)) * 1.4426950408889634f;
+  static int* op_split_cnt = nullptr;   // arrival counters of the last-CTA merge, left at zero by every merge
+  static int op_split_cnt_len = 0;
+  if (splits > 1 && B * nkv > op_split_cnt_len) {
+    B200_CUDA_OK(cudaFree(op_split_cnt));
+    op_split_cnt = nullptr;
+    B200_CUDA_OK(cudaMalloc(reinterpret_cast<void**>(&op_split_cnt), (size_t)B * nkv * sizeof(int)));
+    B200_CUDA_OK(cudaMemset(op_split_cnt, 0, (size_t)B * nkv * sizeof(int)));
+    op_split_cnt_len = B * nkv;
+  }
+  p.split_counter = op_split_cnt;
   return launch_attn_decode(p, B, (cudaStream_t)stream);
 }
 
@@ -2204,8 +2106,8 @@ int b200_op_rope_kv(const void* qkv, int64_t ld, void* q_out, int64_t ldq, void*
   p.qkv = (const bf16*)qkv; p.ld = ld; p.q_out = (bf16*)q_out; p.ldq = ldq; p.kcache = (bf16*)kcache; p.vcache = (bf16*)vcache;
   p.page_table = page_table; p.max_pages = max_pages; p.tok_seq = tok_seq; p.tok_pos = tok_pos;
   p.cos_tab = (const bf16*)cos_tab; p.sin_tab = (const bf16*)sin_tab; p.nh = nh; p.nkv = nkv;
-  p.T = T; p.tokens_per_cta = (getenv("B200_ROPE_TOKENS_PER_CTA") && T >= 4096) ? atoi(getenv("B200_ROPE_TOKENS_PER_CTA")) : 1;
-  rope_kv_kernel<<<(T + p.tokens_per_cta - 1) / p.tokens_per_cta, 512, 0, (cudaStream_t)stream>>>(p);
+  p.T = T;
+  rope_kv_kernel<<<T, 512, 0, (cudaStream_t)stream>>>(p);
   B200_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -4,21 +4,21 @@
 //   warp 1   : MMA issuer    (one thread, tcgen05.mma cta_group::1 kind::f16, fp32 accumulators in TMEM)
 //   warps 2-5: epilogue      (tcgen05.ld -> registers -> fused epilogue -> global), double-buffered TMEM
 //
-// The same kernel serves both phases of the LLM path (SURVEY.md §8a rows 13-17):
-//   * prefill  : A = activations [T,K], B = weight [N_out,K]           -> row-major epilogues
-//   * decode   : A = weight [N_out,K] (M = N_out), B = activations [batch,K] ("swap-AB": the 128-row MMA
-//                M dimension is filled by weight rows, the small batch rides in the MMA N dimension, so no
-//                tensor-core work is wasted on padding and each CTA streams a contiguous weight slab)
-//                -> transposed epilogues, optional split-K with fp32 partials.
+// This kernel is the decode GEMM (SURVEY.md §8a rows 13-17); prefill runs on the 2-CTA kernel (gemm_2cta.cuh).
+// A = weight [N_out,K] (M = N_out), B = activations [batch,K] ("swap-AB": the 128-row MMA M dimension is filled
+// by weight rows, the small batch rides in the MMA N dimension, so no tensor-core work is wasted on padding and
+// each CTA streams a contiguous weight slab) -> transposed epilogues, optional split-K with fp32 partials.
 #pragma once
 #include "common.cuh"
 
 namespace b200 {
 
 enum GemmEpi : int {
+  // row-major epilogues of the 2-CTA prefill kernel
   EPI_STORE = 0,      // out[m][n] = bf16(acc)
   EPI_STORE_RES = 1,  // out[m][n] = bf16(bf16(acc) + residual[m][n])           (o_proj / down_proj + residual)
   EPI_SWIGLU = 2,     // B rows interleaved {16 gate,16 up}: out[m][n/2] = bf16(bf16(silu(g)) * u)
+  // transposed epilogues of the swap-AB decode kernel
   EPI_T_STORE = 3,    // out[n][m] = bf16(acc)                                    (swap-AB)
   EPI_T_SWIGLU = 4,   // A rows interleaved {16 gate,16 up}: out[n][m/2] = ...    (swap-AB)
   EPI_T_PARTIAL = 5,  // ws[split][n][m] = acc (fp32)                             (swap-AB split-K)
@@ -38,7 +38,6 @@ struct GemmParams {
   int out_cols;            // logical number of output columns (bounds for SWIGLU modes = N/2 resp. M/2)
   unsigned long long hint_a, hint_b;
   int prefetch_a;          // A (weights) does not depend on the previous kernel: stream it before griddepcontrol.wait
-  int l2_prefetch_kb;      // additional k-blocks of A to pull into L2 (beyond the smem stages) before the wait
   // sched == 1: "stream-K" — the m_tiles * kb_total k-block iterations are cut into gridDim.x equal contiguous
   // ranges, so every SM streams the same number of weight bytes whatever the tile count (few tiles under tensor
   // parallelism, 224 tiles on 148 SMs, ...).  A tile covered by several CTAs is finished by the CTA that owns
@@ -51,7 +50,7 @@ struct GemmParams {
   const int* m_rt;
   const int* n_rt;
   const int* row_off;      // device row offset of the activation / output rows inside a grouped (per-expert) buffer
-  int swap_ab;             // 1: A is the weight (decode kernels) -> row_off applies to B and to the output rows n
+                           // (2-CTA kernel: rows of A and of the output; swap-AB kernel: rows of B and output rows n)
   // grouped (per-expert) swap-AB problem in ONE launch: A = [groups][M][K] stacked weights, m_tiles = groups * group_m_tiles;
   // tile m_t belongs to group g = m_t / group_m_tiles whose activation rows are row_off[g] .. + n_rt[g] (tiles of
   // empty groups are skipped: their weights are never streamed) and whose outputs start at out + g * group_out_stride
@@ -63,8 +62,6 @@ struct GemmParams {
   bf16* rope_kcache; bf16* rope_vcache;                      // this layer's [page][kv_head][64][128]
   const bf16* rope_cos; const bf16* rope_sin;                // [max_pos][64]
   int rope_nh, rope_nkv;
-  int group_pairs;         // 2-CTA prefill kernel: m-pairs per raster group (0 = default 8)
-  int stream_out;          // 2-CTA prefill kernel: cache-streaming output stores
   int sched;
   int sk_slots;            // partial slots per tile
   float* sk_ws;            // [m_tiles][sk_slots][BLOCK_N][128] fp32
@@ -81,8 +78,8 @@ struct GemmCfg {
   static constexpr int kABytes = kGemmBlockM * kGemmBlockK * 2;  // 16 KB
   static constexpr int kBBytes = BLOCK_N * kGemmBlockK * 2;
   static constexpr int kStageBytes = kABytes + kBBytes;
-  static constexpr int kStages = (BLOCK_N >= 256) ? 4 : (BLOCK_N >= 128 ? 6 : 8);
-  static constexpr int kTmemCols = (2 * BLOCK_N < 32) ? 32 : 2 * BLOCK_N;  // power of two for 16..256
+  static constexpr int kStages = BLOCK_N >= 128 ? 6 : 8;
+  static constexpr int kTmemCols = (2 * BLOCK_N < 32) ? 32 : 2 * BLOCK_N;  // power of two for 16..64
   static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align slack*/ + 256 /*barriers*/;
 };
 
@@ -100,15 +97,12 @@ __device__ __forceinline__ int sk_owner(long long it, long long W, int P) {   //
   return c;
 }
 
-// The work list of CTA `cta` of `ncta`: shared by the GEMM kernel (cta = blockIdx.x) and by the weight-stream
-// prefetcher, which walks the same list ahead of it.
-struct GemmSched { int m_tiles, n_tiles, splits, kb_total, kb_per_split, sched; };
-
-__device__ __forceinline__ bool gemm_get_seg(const GemmSched& p, int idx, GemmSeg& g, int m_tiles_rt, int cta, int ncta) {
+// The work list of this CTA: its idx-th segment
+__device__ __forceinline__ bool gemm_get_seg(const GemmParams& p, int idx, GemmSeg& g, int m_tiles_rt) {
   g.slot = 0;
   if (m_tiles_rt <= 0) return false;
   if (p.sched == 0) {
-    const int u = cta + idx * ncta;
+    const int u = (int)blockIdx.x + idx * (int)gridDim.x;
     if (u >= m_tiles_rt * p.n_tiles * p.splits) return false;
     const int tile = u / p.splits;
     g.split = u - tile * p.splits;
@@ -124,7 +118,7 @@ __device__ __forceinline__ bool gemm_get_seg(const GemmSched& p, int idx, GemmSe
     g.type = 0;
     return true;
   }
-  const int P = ncta, c = cta, KB = p.kb_total;
+  const int P = (int)gridDim.x, c = (int)blockIdx.x, KB = p.kb_total;
   const long long W = (long long)p.m_tiles * KB;
   const long long lo = W * c / P, hi = W * (c + 1) / P;
   if (lo >= hi) return false;
@@ -149,11 +143,6 @@ __device__ __forceinline__ bool gemm_get_seg(const GemmSched& p, int idx, GemmSe
     return true;
   }
   return false;
-}
-
-__device__ __forceinline__ bool gemm_get_seg(const GemmParams& p, int idx, GemmSeg& g, int m_tiles_rt) {
-  const GemmSched sc{p.m_tiles, p.n_tiles, p.splits, p.kb_total, p.kb_per_split, p.sched};
-  return gemm_get_seg(sc, idx, g, m_tiles_rt, (int)blockIdx.x, (int)gridDim.x);
 }
 
 template <int BLOCK_N, int EPI>
@@ -203,9 +192,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
     if (p.n_rt && !gmt) N_rt = min(p.N, *p.n_rt);
   }
   const int m_tiles_rt = gmt ? p.m_tiles : ((M_rt <= 0 || N_rt <= 0) ? 0 : (M_rt + kGemmBlockM - 1) / kGemmBlockM);
-  const int roff = (p.row_off && !gmt) ? *p.row_off : 0;   // (read after the wait above: set together with m_rt / n_rt)
-  const int roff_a = p.swap_ab ? 0 : roff;
-  int roff_b = p.swap_ab ? roff : 0;
+  int roff_b = (p.row_off && !gmt) ? *p.row_off : 0;   // (read after the wait above: set together with m_rt / n_rt)
 
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer
@@ -216,7 +203,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
       GemmSeg sg;
       for (int idx = 0; gemm_get_seg(p, idx, sg, m_tiles_rt); ++idx) {
         const int m_t = sg.m_t, n_t = sg.n_t, kb0 = sg.kb0, kb1 = sg.kb1;
-        int a_row = m_t * kGemmBlockM + roff_a, b_off = roff_b;
+        int a_row = m_t * kGemmBlockM, b_off = roff_b;
         if (gmt) {
           const int g = m_t / gmt;
           if (p.n_rt[g] <= 0) continue;
@@ -234,8 +221,6 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
               mbar_arrive_expect_tx(&full_bar[i], Cfg::kStageBytes);
               tma_load_2d(smem + i * Cfg::kStageBytes, &tmap_a, &full_bar[i], (kb0 + i) * kGemmBlockK, a_row, p.hint_a);
             }
-            const int npf = min(npre + p.l2_prefetch_kb, kb1 - kb0);
-            for (int i = npre; i < npf; ++i) tma_prefetch_l2_2d(&tmap_a, (kb0 + i) * kGemmBlockK, m_t * kGemmBlockM);
             pdl_wait();
             _ts.mark();
             for (int i = 0; i < npre; ++i)
@@ -358,68 +343,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
 #pragma unroll
           for (int j = 0; j < CH; ++j) v[j] += acc[j];
         }
-        if constexpr (EPI == EPI_STORE || EPI == EPI_STORE_RES) {
-          if (m < M_rt) {
-            bf16* orow = reinterpret_cast<bf16*>(p.out) + (long long)(m + roff_a) * p.ldo + n0 + c0;
-            const bf16* rrow = (EPI == EPI_STORE_RES) ? p.residual + (long long)(m + roff_a) * p.ldo + n0 + c0 : nullptr;
-            const bool vec = (nvalid == CH) && ((p.ldo & 7) == 0) && ((reinterpret_cast<uintptr_t>(p.out) & 15) == 0);
-            if (vec) {
-#pragma unroll
-              for (int j = 0; j < CH; j += 8) {
-                float f[8];
-#pragma unroll
-                for (int t = 0; t < 8; ++t) f[t] = v[j + t];
-                if constexpr (EPI == EPI_STORE_RES) {
-                  uint4 rr = *reinterpret_cast<const uint4*>(rrow + j);
-                  const uint32_t rw[4] = {rr.x, rr.y, rr.z, rr.w};
-#pragma unroll
-                  for (int t = 0; t < 4; ++t) {
-                    float2 r2 = unpack_bf16x2(rw[t]);
-                    f[2 * t] = bf16_round(f[2 * t]) + r2.x;
-                    f[2 * t + 1] = bf16_round(f[2 * t + 1]) + r2.y;
-                  }
-                }
-                uint4 o;
-                o.x = pack_bf16x2(f[0], f[1]);
-                o.y = pack_bf16x2(f[2], f[3]);
-                o.z = pack_bf16x2(f[4], f[5]);
-                o.w = pack_bf16x2(f[6], f[7]);
-                *reinterpret_cast<uint4*>(orow + j) = o;
-              }
-            } else {
-              for (int j = 0; j < nvalid; ++j) {
-                float f = v[j];
-                if constexpr (EPI == EPI_STORE_RES) f = bf16_round(f) + __bfloat162float(rrow[j]);
-                orow[j] = __float2bfloat16_rn(f);
-              }
-            }
-          }
-        } else if constexpr (EPI == EPI_SWIGLU) {
-          // columns [c0, c0+16) = gate, [c0+16, c0+32) = up of output columns (n0+c0)/2 + j
-          static_assert(EPI != EPI_SWIGLU || CH == 32, "SWIGLU needs 32-column chunks");
-          if (m < M_rt) {
-            const int oc = (n0 + c0) >> 1;
-            bf16* orow = reinterpret_cast<bf16*>(p.out) + (long long)(m + roff_a) * p.ldo + oc;
-            float h[16];
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-              const float g = bf16_round(v[j]);
-              const float up = bf16_round(v[16 + j]);
-              h[j] = bf16_round(silu_f(g)) * up;
-            }
-            if (oc + 16 <= p.out_cols && (p.ldo & 7) == 0) {
-              uint4 o0, o1;
-              o0.x = pack_bf16x2(h[0], h[1]);   o0.y = pack_bf16x2(h[2], h[3]);
-              o0.z = pack_bf16x2(h[4], h[5]);   o0.w = pack_bf16x2(h[6], h[7]);
-              o1.x = pack_bf16x2(h[8], h[9]);   o1.y = pack_bf16x2(h[10], h[11]);
-              o1.z = pack_bf16x2(h[12], h[13]); o1.w = pack_bf16x2(h[14], h[15]);
-              reinterpret_cast<uint4*>(orow)[0] = o0;
-              reinterpret_cast<uint4*>(orow)[1] = o1;
-            } else {
-              for (int j = 0; j < 16 && oc + j < p.out_cols; ++j) orow[j] = __float2bfloat16_rn(h[j]);
-            }
-          }
-        } else if constexpr (EPI == EPI_T_STORE) {
+        if constexpr (EPI == EPI_T_STORE) {
           if (m < M_rt) {
             bf16* o = reinterpret_cast<bf16*>(p.out) + out_off + (long long)(n0 + c0 + roff_b) * p.ldo + m;
 #pragma unroll

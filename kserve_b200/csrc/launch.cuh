@@ -4,7 +4,6 @@
 #include <map>
 #include <mutex>
 #include <tuple>
-#include <vector>
 
 #include "attention.cuh"
 #include "attention_tc.cuh"
@@ -16,7 +15,6 @@
 #include "moe.cuh"
 #include "cb.cuh"
 #include "sampling.cuh"
-#include "prefetch.cuh"
 
 namespace b200 {
 
@@ -141,16 +139,6 @@ int launch_gemm_2cta_inst(const CUtensorMap* ta, const CUtensorMap* tb, const Ge
   return 0;
 }
 
-// Host side of the weight-stream prefetch (prefetch.cuh): while a decode step is being enqueued, every weight-streaming
-// GEMM takes the next index of the step's table; in `recording` mode (first, eager enqueue of a graph key) its
-// descriptor is appended, in capture mode the engine launches the prefetch of the NEXT table entry beside it.
-struct PfCtx {
-  bool active = false;
-  bool recording = false;
-  int count = 0;            // GEMMs seen so far in this enqueue
-  std::vector<PfGemm> table;
-};
-
 struct GemmArgs {
   const bf16* A; int a_rows;        // rows of the A buffer as declared to TMA (>= M)
   const bf16* B; int b_rows;        // rows of the B buffer as declared to TMA (>= N)
@@ -167,12 +155,8 @@ struct GemmArgs {
   const int* row_off = nullptr;
   int groups = 0;                   // > 0: grouped swap-AB problem (see GemmParams::group_m_tiles); A rows = groups * M,
   long long group_out_stride = 0;   // n_rt / row_off are arrays of `groups` entries
-  PfCtx* pf = nullptr;              // weight-stream prefetcher context of the step being enqueued (decode only)
   const RopeKvParams* rope = nullptr;   // EPI_ROPE_KV: where RoPE(k) / v go and the tables (q is rotated in place in `out`)
 };
-
-// GEMMs whose weight operand depends on nothing the step computes (decode swap-AB, no device-side extents)
-inline bool pf_eligible(const GemmArgs& a) { return a.stream_a && !a.n_rt && !a.m_rt && a.groups == 0 && a.N <= a.block_n; }
 
 inline int launch_gemm(TmapCache& cache, const GemmArgs& a, int num_sms, cudaStream_t s) {
   B200_REQUIRE(a.K % 8 == 0, "K must be a multiple of 8");
@@ -193,34 +177,21 @@ inline int launch_gemm(TmapCache& cache, const GemmArgs& a, int num_sms, cudaStr
   p.out = a.out; p.residual = a.residual; p.ldo = a.ldo; p.split_stride = a.split_stride; p.out_cols = a.out_cols;
   p.hint_a = a.stream_a ? kEvictFirst : kEvictLast;
   p.hint_b = a.stream_a ? kEvictLast : kEvictNormal;
-  p.m_rt = a.m_rt; p.n_rt = a.n_rt; p.row_off = a.row_off; p.swap_ab = a.stream_a ? 1 : 0;
+  p.m_rt = a.m_rt; p.n_rt = a.n_rt; p.row_off = a.row_off;
   p.group_m_tiles = 0; p.group_out_stride = a.group_out_stride;
-  {
-    // r02 (tools/prefill_gemm.py, T = 32768): raster groups of 12 m-pairs + cache-streaming output stores: gate/up 5.47 -> 4.76 ms,
-    // down 3.34 -> 2.57 ms, qkv 1.126 -> 1.108 ms (the 940 MB output stream no longer evicts the A / B tiles other CTAs re-read)
-    static const int gp = getenv("B200_2CTA_GROUP") ? atoi(getenv("B200_2CTA_GROUP")) : 12;
-    static const int cs = getenv("B200_2CTA_CS") ? atoi(getenv("B200_2CTA_CS")) : 1;
-    p.group_pairs = gp; p.stream_out = cs;
-  }
   if (a.groups > 0) {
     B200_REQUIRE(a.stream_a && a.n_rt && a.row_off && !a.m_rt && a.N <= a.block_n, "grouped GEMM: swap-AB with per-group n_rt / row_off");
     p.group_m_tiles = p.m_tiles;
     p.m_tiles *= a.groups;
   }
   p.prefetch_a = (a.stream_a && !a.n_rt && !a.m_rt) ? 1 : 0;
-  {
-    static const int l2pf = getenv("B200_L2_PREFETCH_KB") ? atoi(getenv("B200_L2_PREFETCH_KB")) : 0;
-    p.l2_prefetch_kb = a.stream_a ? l2pf : 0;
-  }
   const int units = p.m_tiles * p.n_tiles * p.splits;
   int grid = units < num_sms ? units : num_sms;
-  static const bool sk_on = getenv("B200_NO_STREAMK") == nullptr;
   p.sched = 0; p.sk_slots = 0; p.sk_ws = a.sk_ws; p.sk_flags = a.sk_flags;
   // only when every tile is cut into at most two pieces (m_tiles >= SMs): finishing many-piece tiles inside the
   // kernel serialises the reduction on the tile owner and measured slower than split-K + a reducing consumer
-  static const bool gu_sk = getenv("B200_GU_STREAMK") != nullptr;
-  const bool sk_any = getenv("B200_STREAMK_ANY") != nullptr || (gu_sk && a.epi == EPI_T_SWIGLU);
-  if (sk_on && a.groups == 0 && a.sk_ws && a.sk_flags && a.stream_a && p.splits == 1 && p.n_tiles == 1 && p.m_tiles <= a.sk_tiles &&
+  const bool sk_any = getenv("B200_STREAMK_ANY") != nullptr;
+  if (a.groups == 0 && a.sk_ws && a.sk_flags && a.stream_a && p.splits == 1 && p.n_tiles == 1 && p.m_tiles <= a.sk_tiles &&
       (p.m_tiles >= num_sms || sk_any) && (p.m_tiles % num_sms) != 0 && (a.epi == EPI_T_STORE || a.epi == EPI_T_SWIGLU)) {
     const long long W = (long long)p.m_tiles * p.kb_total;
     const int g2 = (int)std::min<long long>(num_sms, W);
@@ -230,22 +201,11 @@ inline int launch_gemm(TmapCache& cache, const GemmArgs& a, int num_sms, cudaStr
       p.sched = 1; p.sk_slots = slots; grid = g2;
     }
   }
-  if (a.pf && a.pf->active && pf_eligible(a) && p.n_tiles == 1) {
-    if (a.pf->recording && a.pf->count < kPfMaxGemms) {
-      PfGemm g{};
-      g.tmap_a = *ta;
-      g.sched = GemmSched{p.m_tiles, p.n_tiles, p.splits, p.kb_total, p.kb_per_split, p.sched};
-      g.grid = grid;
-      a.pf->table.push_back(g);
-    }
-    a.pf->count++;
-  }
   B200_REQUIRE(p.splits == 1 || a.epi == EPI_T_PARTIAL, "split-K only with the fp32 partial epilogue");
   p.rope_tok_seq = nullptr; p.rope_tok_pos = nullptr; p.rope_page_table = nullptr; p.rope_max_pages = 0;
   p.rope_kcache = nullptr; p.rope_vcache = nullptr; p.rope_cos = nullptr; p.rope_sin = nullptr; p.rope_nh = 0; p.rope_nkv = 0;
-  const bool use_2cta = getenv("B200_NO_2CTA") == nullptr;
   if (a.epi == EPI_ROPE_KV) {
-    B200_REQUIRE(use_2cta && a.block_n == 256 && a.rope && a.N == (a.rope->nh + 2 * a.rope->nkv) * kHeadDim,
+    B200_REQUIRE(a.block_n == 256 && a.rope && a.N == (a.rope->nh + 2 * a.rope->nkv) * kHeadDim,
                  "EPI_ROPE_KV is the 2-CTA prefill QKV projection");
     p.rope_tok_seq = a.rope->tok_seq; p.rope_tok_pos = a.rope->tok_pos; p.rope_page_table = a.rope->page_table;
     p.rope_max_pages = a.rope->max_pages; p.rope_kcache = a.rope->kcache; p.rope_vcache = a.rope->vcache;
@@ -255,7 +215,7 @@ inline int launch_gemm(TmapCache& cache, const GemmArgs& a, int num_sms, cudaStr
     if (rc2) return rc2;
     return launch_gemm_2cta_inst<EPI_ROPE_KV>(ta, tb2, p, num_sms, s);
   }
-  if (use_2cta && a.block_n == 256 && a.epi <= EPI_SWIGLU) {
+  if (a.block_n == 256 && a.epi <= EPI_SWIGLU) {
     const CUtensorMap* tb2;
     int rc2 = cache.get(a.B, a.b_rows, a.K, 128, &tb2);   // each CTA of the pair stages half of the 256 weight rows
     if (rc2) return rc2;
@@ -265,9 +225,6 @@ inline int launch_gemm(TmapCache& cache, const GemmArgs& a, int num_sms, cudaStr
   }
 #define B200_GEMM_CASE(BN, E) \
   if (a.block_n == BN && a.epi == E) return launch_gemm_inst<BN, E>(ta, tb, p, grid, s);
-  B200_GEMM_CASE(256, EPI_STORE)
-  B200_GEMM_CASE(256, EPI_STORE_RES)
-  B200_GEMM_CASE(256, EPI_SWIGLU)
   B200_GEMM_CASE(16, EPI_T_STORE)
   B200_GEMM_CASE(16, EPI_T_SWIGLU)
   B200_GEMM_CASE(16, EPI_T_PARTIAL)
@@ -307,8 +264,7 @@ inline int launch_rmsnorm(int mode, bf16* x, const bf16* w, bf16* xn, int rows, 
   const float* np = nullptr;
   const bf16* ny = nullptr;
   // prefill-sized launches of the plain / post-all-reduce norm: the warp-per-row kernel
-  static const bool rows_off = getenv("B200_NORM_ROWS_OFF") != nullptr;
-  if (!rows_off && mode != 1 && rows >= 256) {
+  if (mode != 1 && rows >= 256) {
 #define B200_NORM_ROWS(NVV)                                                                                                       \
     if (H == NVV * 256) {                                                                                                          \
       if (mode == 0) B200_CUDA_OK(launch_k(rmsnorm_rows_kernel<0, NVV>, dim3((rows + 7) / 8), dim3(256), 0, s, x, w, xn, rows, eps, ny)); \
@@ -324,19 +280,7 @@ inline int launch_rmsnorm(int mode, bf16* x, const bf16* w, bf16* xn, int rows, 
   return 0;
 }
 
-constexpr int kPrefillSmem = 5 * kTileBytes;
 constexpr int kDecodeSmem = 4096 + 2 * kDecStages * kTileBytes + 10 * kHeadDim * 4 + 2 * kHeadDim * 2;
-
-inline int launch_attn_prefill(const AttnPrefillParams& p, int B, int max_len, cudaStream_t s) {
-  static bool configured = false;
-  if (!configured) {
-    B200_CUDA_OK(cudaFuncSetAttribute(attn_prefill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPrefillSmem));
-    configured = true;
-  }
-  dim3 grid((max_len + 63) / 64, p.nh, B);
-  B200_CUDA_OK(launch_k(attn_prefill_kernel, grid, dim3(kAttnThreads), kPrefillSmem, s, p));
-  return 0;
-}
 
 // tcgen05 prefill attention: q rows [q_rows][ldq] (head h at column h*128), paged caches [num_pages][nkv][64][128]
 inline int launch_attn_prefill_tc(TmapCache& cache, const bf16* q, int q_rows, long long ldq, const bf16* kcache,
@@ -364,11 +308,9 @@ inline int launch_attn_decode(const AttnDecodeParams& p, int B, cudaStream_t s) 
     configured = true;
   }
   B200_REQUIRE(p.G >= 1 && p.G <= 8, "GQA group size must be in [1, 8]");
+  B200_REQUIRE(p.splits == 1 || p.split_counter, "split decode attention needs the arrival counters of its merge");
   dim3 grid(B * p.nkv, p.splits);
   B200_CUDA_OK(launch_k(attn_decode_kernel, grid, dim3(kAttnThreads), kDecodeSmem, s, p));
-  if (p.splits > 1 && !p.split_counter) {
-    B200_CUDA_OK(launch_k(attn_combine_kernel, dim3(B * p.nh), dim3(128), 0, s, (const float*)p.part_o, (const float*)p.part_ml, p.out, p.ldo, p.nkv, p.G, p.splits));
-  }
   return 0;
 }
 

@@ -228,14 +228,12 @@ moe_place_gather_kernel(const bf16* __restrict__ xn, const int32_t* __restrict__
   }
 }
 
-// Combine + residual + next RMSNorm.  Expert outputs are either bf16 rows yg[row][H] (prefill) or fp32 split-K
-// partials part[e][split][n][H] with n = row - off[e] (decode).  TP: writes the per-rank partial sum to `ysum`
-// instead (the caller all-reduces it and applies the residual / norm afterwards).
+// Combine + residual + next RMSNorm over the bf16 expert output rows yg[row][H].  TP: writes the per-rank partial
+// sum to `ysum` instead (the caller all-reduces it and applies the residual / norm afterwards).
 struct MoeCombineParams {
   bf16* x; const bf16* w; bf16* xn; int H; float eps;
-  const int32_t* tok_expert; const float* tok_weight; const int32_t* tok_row; const int32_t* off;
+  const int32_t* tok_expert; const float* tok_weight; const int32_t* tok_row;
   const bf16* yg;
-  const float* part; int splits; long long expert_stride, split_stride;   // part + e*expert_stride + s*split_stride + n*H
   bf16* ysum;   // non-null under tensor parallelism
 };
 
@@ -260,21 +258,14 @@ __global__ void __launch_bounds__(kNormThreads) moe_combine_norm_kernel(const Mo
   float ss = 0.f;
   for (int i = threadIdx.x * 8; i < H; i += blockDim.x * 8) {
     float ya[8], yb[8];
-    if (p.part) {
-      sum_partials8(p.part + (long long)ea * p.expert_stride + (long long)(ra - p.off[ea]) * H + i, p.splits, p.split_stride, ya);
-      sum_partials8(p.part + (long long)eb * p.expert_stride + (long long)(rb - p.off[eb]) * H + i, p.splits, p.split_stride, yb);
+    const uint4 ua = *reinterpret_cast<const uint4*>(p.yg + (long long)ra * H + i);
+    const uint4 ub = *reinterpret_cast<const uint4*>(p.yg + (long long)rb * H + i);
+    const uint32_t aw[4] = {ua.x, ua.y, ua.z, ua.w}, bw[4] = {ub.x, ub.y, ub.z, ub.w};
 #pragma unroll
-      for (int t = 0; t < 8; ++t) { ya[t] = bf16_round(ya[t]); yb[t] = bf16_round(yb[t]); }
-    } else {
-      const uint4 ua = *reinterpret_cast<const uint4*>(p.yg + (long long)ra * H + i);
-      const uint4 ub = *reinterpret_cast<const uint4*>(p.yg + (long long)rb * H + i);
-      const uint32_t aw[4] = {ua.x, ua.y, ua.z, ua.w}, bw[4] = {ub.x, ub.y, ub.z, ub.w};
-#pragma unroll
-      for (int t = 0; t < 4; ++t) {
-        const float2 a2 = unpack_bf16x2(aw[t]), b2 = unpack_bf16x2(bw[t]);
-        ya[2 * t] = a2.x; ya[2 * t + 1] = a2.y;
-        yb[2 * t] = b2.x; yb[2 * t + 1] = b2.y;
-      }
+    for (int t = 0; t < 4; ++t) {
+      const float2 a2 = unpack_bf16x2(aw[t]), b2 = unpack_bf16x2(bw[t]);
+      ya[2 * t] = a2.x; ya[2 * t + 1] = a2.y;
+      yb[2 * t] = b2.x; yb[2 * t + 1] = b2.y;
     }
     float f[8];
 #pragma unroll

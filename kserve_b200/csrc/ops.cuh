@@ -262,7 +262,7 @@ struct RopeKvParams {
   const int32_t* tok_pos;                // [T] position within the sequence
   const bf16* cos_tab; const bf16* sin_tab;  // [max_pos][64]
   int nh, nkv;
-  int T, tokens_per_cta;                     // tokens in this launch; consecutive tokens handled by one CTA
+  int T;                                 // tokens in this launch (one CTA each)
 };
 
 __device__ __forceinline__ void load8(const RopeKvParams& p, int t, int col, float (&f)[8]) {
@@ -296,9 +296,7 @@ __global__ void __launch_bounds__(512) rope_kv_kernel(const RopeKvParams p) {
   _ts.mark();
   const int rope_items = (p.nh + p.nkv) * 8;   // 8 threads per roped head (each 8 dims of both halves)
   const int copy_items = p.nkv * 16;           // 16 threads per V head
-  // tokens_per_cta consecutive tokens per CTA (prefill launches: fewer, longer-lived CTAs — the one-token-per-CTA launch
-  // of 32768 CTAs was launch-rate bound at 0.37 of the HBM peak, r01 ncu)
-  for (int t = blockIdx.x * p.tokens_per_cta; t < min(p.T, (int)(blockIdx.x + 1) * p.tokens_per_cta); ++t) {
+  for (int t = blockIdx.x; t < p.T; t += gridDim.x) {   // launched with one CTA per token
   const int pos = p.tok_pos[t];
   const int seq = p.tok_seq[t];
   const int page = p.page_table[(long long)seq * p.max_pages + pos / kPageTokens];

@@ -227,31 +227,9 @@ def _attn_ref(q, k, v, causal_offset=None):
 
 
 @pytest.mark.parametrize("nh,nkv", [(4, 2), (8, 2), (8, 8), (32, 8)])
-@pytest.mark.parametrize("lens", [[5], [64, 1, 130], [200, 63, 65, 128]])
-def test_attn_prefill(lib, nh, nkv, lens):
-    B = len(lens)
-    kc, vc, pt, max_pages, kd, vd = _build_cache(B, lens, nkv, seed=11)
-    T = sum(lens)
-    q = _rand(T, nh * 128, seed=12)
-    out = torch.zeros((T, nh * 128), dtype=torch.bfloat16, device=DEV)
-    cu = torch.tensor([0] + list(torch.tensor(lens).cumsum(0)), dtype=torch.int32, device=DEV)
-    slot = torch.arange(B, dtype=torch.int32, device=DEV)
-    _check(lib, lib.b200_op_attn_prefill(_ptr(q), nh * 128, _ptr(out), nh * 128, _ptr(kc), _ptr(vc), _ptr(pt), max_pages,
-                                         _ptr(cu), _ptr(slot), B, max(lens), nh, nkv, None), "attn_prefill")
-    torch.cuda.synchronize()
-    t0 = 0
-    for b, l in enumerate(lens):
-        qb = q[t0:t0 + l].view(l, nh, 128).transpose(0, 1)
-        ref = _attn_ref(qb, kd[b, :, :l], vd[b, :, :l], causal_offset=0)
-        # P is rounded to bf16 before PV (as flash kernels do): ~2^-8 relative on O(1) values
-        _cmp(f"attn_prefill b{b} len{l}", out[t0:t0 + l], ref, 2e-2, 2e-2)
-        t0 += l
-
-
-@pytest.mark.parametrize("nh,nkv", [(4, 2), (8, 2), (32, 8)])
 @pytest.mark.parametrize("lens", [[5], [64, 1, 130], [200, 63, 65, 128, 129], [700, 257]])
 def test_attn_prefill_tcgen05(lib, nh, nkv, lens):
-    """The tcgen05 / TMEM prefill attention (engine default) against the fp32 statement of causal GQA attention."""
+    """The tcgen05 / TMEM prefill attention (the engine's) against the fp32 statement of causal GQA attention."""
     B = len(lens)
     kc, vc, pt, max_pages, kd, vd = _build_cache(B, lens, nkv, seed=21)
     T = sum(lens)
@@ -277,22 +255,23 @@ def test_attn_decode(lib, nh, nkv, splits):
     B = len(lens)
     kc, vc, pt, max_pages, kd, vd = _build_cache(B, lens, nkv, seed=13)
     q = _rand(B, nh * 128, seed=14)
-    out = torch.zeros((B, nh * 128), dtype=torch.bfloat16, device=DEV)
     slot = torch.arange(B, dtype=torch.int32, device=DEV)
     pos = torch.tensor([l - 1 for l in lens], dtype=torch.int32, device=DEV)
     G = nh // nkv
     po = torch.zeros((B * nkv * splits * G * 128,), dtype=torch.float32, device=DEV)
     pml = torch.zeros((B * nkv * splits * G * 2,), dtype=torch.float32, device=DEV)
-    _check(lib, lib.b200_op_attn_decode(_ptr(q), nh * 128, _ptr(out), nh * 128, _ptr(kc), _ptr(vc), _ptr(pt), max_pages,
-                                        _ptr(slot), _ptr(pos), B, nh, nkv, splits, _ptr(po), _ptr(pml), None), "attn_decode")
-    torch.cuda.synchronize()
-    for b, l in enumerate(lens):
-        qb = q[b].view(nh, 1, 128)
-        ref = _attn_ref(qb, kd[b, :, :l], vd[b, :, :l])
-        _cmp(f"attn_decode b{b} len{l} splits{splits}", out[b:b + 1], ref, 2e-2, 2e-2)
+    for rep in range(2):   # splits > 1: the last-CTA merge must leave its arrival counters at zero for the next call
+        out = torch.zeros((B, nh * 128), dtype=torch.bfloat16, device=DEV)
+        _check(lib, lib.b200_op_attn_decode(_ptr(q), nh * 128, _ptr(out), nh * 128, _ptr(kc), _ptr(vc), _ptr(pt), max_pages,
+                                            _ptr(slot), _ptr(pos), B, nh, nkv, splits, _ptr(po), _ptr(pml), None), "attn_decode")
+        torch.cuda.synchronize()
+        for b, l in enumerate(lens):
+            qb = q[b].view(nh, 1, 128)
+            ref = _attn_ref(qb, kd[b, :, :l], vd[b, :, :l])
+            _cmp(f"attn_decode rep{rep} b{b} len{l} splits{splits}", out[b:b + 1], ref, 2e-2, 2e-2)
 
 
-@pytest.mark.parametrize("T", [70, 4101])      # >= 4096 tokens: four consecutive tokens per CTA
+@pytest.mark.parametrize("T", [70, 4101])      # 4101 tokens: 66 shuffled pages, one CTA per token
 def test_rope_kv(lib, T):
     from kserve_b200.engine import hf_rope_tables
     nh, nkv = 4, 2

@@ -12,7 +12,7 @@ from bench import MODELS, gpu_weights  # noqa: E402
 from kserve_b200 import _lib  # noqa: E402
 from kserve_b200.engine import B200Engine  # noqa: E402
 
-KIND = {1: "gemm", 2: "rmsnorm", 3: "rope", 4: "attn_dec", 5: "attn_comb", 6: "argmax", 7: "step", 8: "embed", 9: "attn_pre", 10: "other", 11: "prefetch"}
+KIND = {1: "gemm", 2: "rmsnorm", 3: "rope", 4: "attn_dec", 6: "argmax", 7: "step", 8: "embed", 9: "attn_pre", 10: "other"}
 EPI = {3: "T_STORE", 4: "T_SWIGLU", 5: "T_PARTIAL", 0: "STORE", 1: "STORE_RES", 2: "SWIGLU"}
 
 
